@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the per-frame inference hot path (BASELINE.json metric: frames/s @256x256, bs16).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 16] [--size 256]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 16] [--size 256] [--dump-outputs DIR]
 
 One *step* = one pass of the hot path over one batch of B synthetic target frames per GPU:
 fused correspondence (raster + cond + T + image warp) -> ImpersonatorGenerator.inference on the
@@ -17,6 +17,9 @@ no per-step collective.  Prints ONE JSON line on rank 0.
             same ATen CPU ops the reference modules call) on the host cores, bounded sample, rank 0, N=1.
 ``--impl reference`` times that CPU path as the reference arm (the reference tree itself does not exist
             on the GPU box; its CUDA rasterizer has no CPU path at all).
+``--dump-outputs DIR`` writes what the last timed step returned -- the generated frames, float32 [B,3,H,W] -- as
+            DIR/pred.npy (rank 0's frames; the first frames only beyond DUMP_BYTES).  The inputs are seeded, so two builds
+            run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -32,6 +35,7 @@ sys.path.insert(0, ROOT)
 
 FLOPS_PER_FRAME_TC = None   # filled from the conv plans (algorithmic 2*MAC of the tensor-core layers)
 REF_INFERENCE_GFLOP = 105.579   # BASELINE.md section 2: generator.inference per frame @256^2
+DUMP_BYTES = 64 << 20           # --dump-outputs writes at most this much
 
 
 def parse():
@@ -47,6 +51,7 @@ def parse():
     ap.add_argument("--profile-range", action="store_true", help="cudaProfilerStart/Stop around the timed steps (ncu --profile-from-start off)")
     ap.add_argument("--steady-steps", type=int, default=400, help="length of the extra steady-state leg (N=1; 0 = skip)")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of one step (outside the timed region)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frames the last timed step returned as DIR/pred.npy")
     return ap.parse_args()
 
 
@@ -380,9 +385,12 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last_out = [None]
+
     def timed(fn, steps, warmup, collective=True, profile=False):
         """collective=False: rank-local timing (the rank-0-only extras must not enter a barrier).  profile: bracket the
-        timed steps with cudaProfilerStart/Stop (--profile-range, for `ncu --profile-from-start off`)."""
+        timed steps with cudaProfilerStart/Stop (--profile-range, for `ncu --profile-from-start off`).  The last step's
+        output is left in last_out[0]."""
         for i in range(warmup):
             fn(i)
         if collective:
@@ -395,7 +403,7 @@ def main():
             torch.cuda.profiler.start()
         e0.record()
         for i in range(steps):
-            fn(warmup + i)
+            last_out[0] = fn(warmup + i)
         e1.record()
         torch.cuda.synchronize()
         if profile:
@@ -422,6 +430,12 @@ def main():
     ms, launches = timed(step_device, args.steps, max(args.warmup, 3), profile=args.profile_range)
     clocks = sampler.stop() if rank == 0 else None
     fps = world * B * args.steps / (ms * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        # copied now: a captured step returns a static buffer that the legs below overwrite
+        import numpy as np
+        pred = last_out[0].float().cpu().numpy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "pred.npy"), pred[:DUMP_BYTES // pred[0].nbytes])
     # ---- BASELINE configs[3] as written: a 64-frame stream sharded over the ranks (8 per GPU at N = 8), strong scaling:
     # total work fixed, every rank runs its 64 / N frames in chunks of at most B; time = max over ranks
     c3_frames = 64

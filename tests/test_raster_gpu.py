@@ -1,6 +1,9 @@
 """GPU parity of the rasterizer / correspondence kernels (through the C ABI) against
-  * the reference's own CUDA kernels compiled for sm_100a (oracle/_ref, bit-exact fim), and
+  * the reference's own CUDA kernels compiled for sm_100a (oracle/_ref, bit-exact fim): SHA-256 digests of their outputs
+    on the inputs of REF_FACES / REF_CASES, stored by tests/golden/make_raster_golden.py, and
   * the C restatement (oracle/raster_ref.c) + torch glue restatement (oracle/nmr_ref.py)."""
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -27,23 +30,20 @@ def run_mine(faces, size, flip=False, want_inv=True):
     return fim, wim, depth, finv
 
 
-def bits(t):
-    return t.contiguous().view(torch.int32)
+def digest(t):
+    return hashlib.sha256(t.detach().cpu().contiguous().numpy().tobytes()).hexdigest()
 
 
-def compare_with_gpu_ref(faces, size):
-    if not raster.gpu_ref_available():
-        pytest.skip("oracle/_ref/libnmr_ref.so not built (reference absent at build time)")
+def compare_with_gpu_ref(case, faces, size):
+    """Bitwise comparison with the outputs of the reference kernels for the faces of REF_FACES[case] at ``size``."""
+    want = json.load(open(os.path.join(GOLD, "raster_ref.json")))["%s@%d" % (case, size)]
+    assert digest(faces) == want["faces"], "the faces differ from those the reference kernels were run on"
     fim, wim, depth, finv = run_mine(faces, size)
-    rfim, rwim, rdepth, rfinv = raster.forward_face_index_map_gpu_ref(faces, size)
-    n_inv = int((bits(finv) != bits(rfinv)).sum())
-    n_fim = int((fim != rfim).sum())
-    n_w = int((bits(wim) != bits(rwim)).sum())
-    n_d = int((bits(depth) != bits(rdepth)).sum())
-    print("covered %d  mismatches: faces_inv %d  fim %d  wim %d  depth %d" % (int((rfim >= 0).sum()), n_inv, n_fim, n_w, n_d))
-    assert n_inv == 0, "faces_inv differs bitwise from the reference kernel_1"
-    assert n_fim == 0, "face_index_map differs from the reference kernel_2"
-    assert n_w == 0 and n_d == 0
+    covered = int((fim >= 0).sum())
+    print("covered %d (reference %d)" % (covered, want["covered"]))
+    assert digest(finv) == want["faces_inv"], "faces_inv differs bitwise from the reference kernel_1"
+    assert covered == want["covered"] and digest(fim) == want["fim"], "face_index_map differs from the reference kernel_2"
+    assert digest(wim) == want["wim"] and digest(depth) == want["depth"]
     return fim
 
 
@@ -56,16 +56,16 @@ def sphere_faces(B, seed, dev):
 def test_sphere_bit_exact_vs_reference_kernels(cuda):
     faces, _, _, _ = sphere_faces(3, 1234, cuda)
     for size in (256, 64):
-        fim = compare_with_gpu_ref(faces, size)
+        fim = compare_with_gpu_ref("sphere_b3_seed1234", faces, size)
         assert int((fim >= 0).sum()) > 100
 
 
 def test_sphere_512_bit_exact(cuda):
     faces, _, _, _ = sphere_faces(2, 77, cuda)
-    compare_with_gpu_ref(faces, 512)
+    compare_with_gpu_ref("sphere_b2_seed77", faces, 512)
 
 
-def test_teapot_batch_with_degenerate_meshes(cuda):
+def teapot_batch_faces():
     """tests/utils.py:11-27 (to_minibatch): the teapot sits in slot 2 of a batch of 4, the other
     three meshes are all-zero vertices -> every face degenerate (whole-image scan path)."""
     g = np.load(os.path.join(GOLD, "teapot.npz"))
@@ -76,8 +76,12 @@ def test_teapot_batch_with_degenerate_meshes(cuda):
     width = torch.tan(torch.tensor(30. / 180 * np.pi))
     zv = torch.stack((zero_v[..., 0] / z / width, zero_v[..., 1] / z / width, z), dim=2)
     zf = zv[0][torch.zeros(tp.shape[0], 3, dtype=torch.long)]
-    faces = torch.stack([zf, zf, tp, zf]).to(cuda).contiguous()
-    fim = compare_with_gpu_ref(faces, 256)
+    return torch.stack([zf, zf, tp, zf]).contiguous()
+
+
+def test_teapot_batch_with_degenerate_meshes(cuda):
+    g = np.load(os.path.join(GOLD, "teapot.npz"))
+    fim = compare_with_gpu_ref("teapot_batch", teapot_batch_faces().to(cuda), 256)
     sil = np.unpackbits(g["silhouette"]).reshape(256, 256).astype(bool)
     mine = (fim[2].flip(0) >= 0).cpu().numpy()
     assert (mine != sil).sum() == 0                      # test_rasterize_silhouettes.py:16-35
@@ -103,20 +107,24 @@ def random_soup(B, F, seed):
 
 def test_random_triangle_soup_bit_exact(cuda):
     for seed, size in ((1, 128), (2, 256), (3, 96)):
-        compare_with_gpu_ref(random_soup(2, 3000, seed).to(cuda), size)
+        compare_with_gpu_ref("soup_seed%d" % seed, random_soup(2, 3000, seed).to(cuda), size)
 
 
-def test_big_faces_bit_exact_and_grid_wide(cuda):
-    """Many faces covering thousands of pixels each (boxes > kBigBox go to the grid-wide scan instead of one warp): bit-exact
-    against the reference kernels, and not a straggler."""
+def big_faces():
     g = torch.Generator().manual_seed(11)
     B, F = 2, 1500
     c = torch.rand(B, F, 1, 2, generator=g) * 1.6 - 0.8
     size = 0.2 + torch.rand(B, F, 1, 1, generator=g) * 1.2                 # 25..180 px wide at 256^2
     xy = c + (torch.rand(B, F, 3, 2, generator=g) - 0.5) * size
     z = 1.0 + torch.rand(B, F, 3, 1, generator=g) * 3
-    faces = torch.cat([xy, z], dim=-1).float().contiguous().to(cuda)
-    compare_with_gpu_ref(faces, 256)
+    return torch.cat([xy, z], dim=-1).float().contiguous()
+
+
+def test_big_faces_bit_exact_and_grid_wide(cuda):
+    """Many faces covering thousands of pixels each (boxes > kBigBox go to the grid-wide scan instead of one warp): bit-exact
+    against the reference kernels, and not a straggler."""
+    faces = big_faces().to(cuda)
+    compare_with_gpu_ref("big_faces", faces, 256)
     for _ in range(3):
         run_mine(faces, 256, want_inv=False)
     torch.cuda.synchronize()
@@ -129,6 +137,14 @@ def test_big_faces_bit_exact_and_grid_wide(cuda):
     ms = e0.elapsed_time(e1) / 10
     print("3000 large faces (avg box ~10^4 px) @256^2: %.3f ms" % ms)
     assert ms < 5.0
+
+
+# the inputs (CPU faces) and image sizes the bit-exact tests above compare on
+REF_FACES = {"sphere_b3_seed1234": lambda: sphere_faces(3, 1234, "cpu")[0], "sphere_b2_seed77": lambda: sphere_faces(2, 77, "cpu")[0],
+             "teapot_batch": teapot_batch_faces, "big_faces": big_faces,
+             **{"soup_seed%d" % s: (lambda s=s: random_soup(2, 3000, s)) for s in (1, 2, 3)}}
+REF_CASES = [("sphere_b3_seed1234", 256), ("sphere_b3_seed1234", 64), ("sphere_b2_seed77", 512), ("teapot_batch", 256),
+             ("soup_seed1", 128), ("soup_seed2", 256), ("soup_seed3", 96), ("big_faces", 256)]
 
 
 def test_flip_rows_matches_torch_flip(cuda):

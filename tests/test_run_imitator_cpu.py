@@ -1,26 +1,53 @@
-"""tests/run_imitator_body.py must be the reference's run_imitator.py main block, character for character (checked where the
-reference tree exists; the GPU box runs the committed copy)."""
+"""tests/run_imitator_body.py must be the reference's run_imitator.py main block, character for character, and the lookup
+tables of impersonator_b200.mesh must equal the reference's utils/mesh.py ones: both checked against digests of the
+reference's own text / outputs, stored by tests/golden/make_run_imitator_golden.py."""
+import hashlib
+import json
 import os
 
+import numpy as np
 import pytest
 
 from run_imitator_body import BODY
 
-REF = "/root/reference/run_imitator.py"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "run_imitator.json")
+MAPPER = "assets/pretrains/mapper.txt"
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree not present (GPU box)")
+def sha256(data):
+    return hashlib.sha256(data).hexdigest()
+
+
+def table_digests(M):
+    """Digests of the tables a utils/mesh.py-style module ``M`` builds from the asset files under the cwd (the ones
+    models/imitator.py:39-41 and models/swapper.py:34-37 use); 'raises AssertionError' where it refuses."""
+    def arr(a):
+        return "%s%s:%s" % (a.dtype, a.shape, sha256(np.ascontiguousarray(a).tobytes()))
+
+    def ids(x):
+        return sha256(json.dumps(x).encode())
+    out = {"mapper.txt": sha256(open(MAPPER, "rb").read())}
+    for name in ("uv_seg", "front", "back", "head", "uv", "seg", "par"):
+        for fb in (False, True):
+            try:
+                out["%s fill_back=%d" % (name, fb)] = arr(M.create_mapping(name, MAPPER, contain_bg=True, fill_back=fb))
+            except AssertionError:
+                out["%s fill_back=%d" % (name, fb)] = "raises AssertionError"
+    for fb in (False, True):
+        parts = M.get_part_face_ids('par', MAPPER, fill_back=fb)
+        out["par ids fill_back=%d" % fb] = ids([[k, [int(i) for i in parts[k]]] for k in parts])
+        for kind in ('head_front', 'head_back'):
+            out["%s ids fill_back=%d" % (kind, fb)] = ids(sorted(int(i) for i in M.get_part_face_ids(kind, MAPPER, fill_back=fb)))
+    return out
+
+
 def test_body_is_the_reference_main_block():
-    src = open(REF).read()
-    main = src[src.index('if __name__ == "__main__":'):]
-    main = main[main.index("\n") + 1:]
-    assert main.rstrip("\n") == BODY.rstrip("\n")
+    assert sha256(BODY.rstrip("\n").encode()) == json.load(open(GOLD))["main_block"]
 
 
 def test_renderer_tables_from_asset_files(tmp_path, monkeypatch):
     """SMPLRenderer(image_size, tex_size, has_front, fill_back=False) as models/imitator.py:39-41 calls it: faces + lookup
     tables come from the files under assets/pretrains (synthetic files in the real formats here)."""
-    import numpy as np
     from impersonator_b200 import mesh, synthetic as S
     from impersonator_b200.nmr import SMPLRenderer
     S.write_synthetic_assets(str(tmp_path), n_targets=1)
@@ -30,32 +57,13 @@ def test_renderer_tables_from_asset_files(tmp_path, monkeypatch):
     assert r.map_fn[-1].tolist() == [0.0, 0.0, 1.0] and float(r.map_fn[:-1, 2].abs().max()) == 0.0
     assert float(r.front_map_fn.sum()) == 500.0 and float(r.back_map_fn.sum()) == 700.0      # head minus front
     assert mesh.get_map_fn_dim('uv_seg') == 3
-    if os.path.exists("/root/reference/utils/mesh.py"):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("ref_mesh", "/root/reference/utils/mesh.py")
-        R = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(R)
-        for name in ("uv_seg", "front", "back", "head", "uv", "seg"):
-            for fb in (False, True):
-                mine = mesh.create_mapping(name, "assets/pretrains/mapper.txt", contain_bg=True, fill_back=fb)
-                ref = R.create_mapping(name, "assets/pretrains/mapper.txt", contain_bg=True, fill_back=fb)
-                assert mine.dtype == ref.dtype and np.array_equal(mine, ref), (name, fb)
-        for fb in (False, True):                                  # the Swapper's tables (models/swapper.py:34-37)
-            if fb:                                                # upstream's 'par' table does not support fill_back either
-                for fn in (mesh.create_mapping, R.create_mapping):
-                    with pytest.raises(AssertionError):
-                        fn('par', "assets/pretrains/mapper.txt", contain_bg=True, fill_back=True)
-            else:
-                mine = mesh.create_mapping('par', "assets/pretrains/mapper.txt", contain_bg=True, fill_back=False)
-                ref = R.create_mapping('par', "assets/pretrains/mapper.txt", contain_bg=True, fill_back=False)
-                assert mine.shape == ref.shape == (13776 + 1, 11) and np.array_equal(mine, ref)
-            mine_ids = mesh.get_part_face_ids('par', "assets/pretrains/mapper.txt", fill_back=fb)
-            ref_ids = R.get_part_face_ids('par', "assets/pretrains/mapper.txt", fill_back=fb)
-            assert list(mine_ids.keys()) == list(ref_ids.keys())
-            assert all(list(mine_ids[k]) == list(ref_ids[k]) for k in ref_ids), fb
-            for kind in ('head_front', 'head_back'):
-                assert sorted(mesh.get_part_face_ids(kind, "assets/pretrains/mapper.txt", fill_back=fb)) == \
-                    sorted(R.get_part_face_ids(kind, "assets/pretrains/mapper.txt", fill_back=fb)), (kind, fb)
+    assert mesh.create_mapping('par', MAPPER, contain_bg=True, fill_back=False).shape == (13776 + 1, 11)
+    with pytest.raises(AssertionError):                           # upstream's 'par' table does not support fill_back either
+        mesh.create_mapping('par', MAPPER, contain_bg=True, fill_back=True)
+    want = json.load(open(GOLD))["tables"]
+    got = table_digests(mesh)
+    assert got["mapper.txt"] == want["mapper.txt"], "the synthetic mapper.txt differs from the one the reference read"
+    assert got == want, sorted(k for k in want if got.get(k) != want[k])
 
 
 def test_networks_factory_names():
